@@ -487,6 +487,26 @@ class Job:
         return {n: (self.d_best[n][:self.counts[n] * 16].clone(), self.d_satd[n].clone(), self.d_sum[n].clone(), self.d_last[n].clone(), self.d_q[n].clone()) for n in SIZES}
 
 
+DUMP_Q_VALUES = 1 << 20      # levels kept per block size in --dump-outputs: a seeded sample of whole blocks
+
+
+def dump_outputs(job, out_dir, V):
+    """what a caller of the step receives for its last picture, per block size: best vector records, SATD ring costs, TU summaries and the
+    levels of a fixed sample of blocks (all of them would be 133 MB as float32); integers stored exactly (float64 where they may pass 2^24)"""
+    os.makedirs(out_dir, exist_ok=True)
+    for n in SIZES:
+        nb = job.counts[n]
+        best = np.frombuffer(job.d_best[n][:nb * 16].cpu().numpy().tobytes(), dtype=V.BEST_DT)
+        np.save(os.path.join(out_dir, 'best_%dx%d.npy' % (n, n)), np.stack([best[f].astype(np.float64) for f in ('dx', 'dy', 'sad', 'cost')], axis=1))
+        np.save(os.path.join(out_dir, 'satd_%dx%d.npy' % (n, n)), job.d_satd[n][:nb * len(refine_pattern())].cpu().numpy().astype(np.float64).reshape(nb, -1))
+        tu = [job.d_sum[n][:nb], job.d_last[n][:nb], job.d_nr[n][:nb]]
+        np.save(os.path.join(out_dir, 'tu_sum_last_rdoq_%dx%d.npy' % (n, n)), np.stack([t.cpu().numpy().astype(np.float64) for t in tu], axis=1))
+        pick = np.sort(np.random.RandomState(n).choice(nb, size=min(nb, DUMP_Q_VALUES // (n * n)), replace=False))
+        q = job.d_q[n][:nb * n * n].cpu().numpy().reshape(nb, n * n)[pick]
+        np.save(os.path.join(out_dir, 'q_%dx%d.npy' % (n, n)), q.astype(np.float32))
+        np.save(os.path.join(out_dir, 'q_blocks_%dx%d.npy' % (n, n)), pick.astype(np.float64))
+
+
 def sharded_parity(env, jobs_all_bands, gather, po, pr, own_job):
     """rank 0: every band recomputed on this GPU alone must equal what the band's owner sent through the all-gather, bit for bit"""
     torch, eng = env['torch'], env['eng']
@@ -603,7 +623,7 @@ def strong_4320p(env, rank, world, pictures=6):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=20, help='timed steps of the headline measurement (the e2e leg times min(max(steps, 2), 5) steps)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--cpu-budget', type=float, default=12.0)
@@ -612,7 +632,12 @@ def main():
     ap.add_argument('--skip-cpu', action='store_true', help='profiling runs: no CPU baseline leg')
     ap.add_argument('--skip-extras', action='store_true', help='profiling runs: no per-kernel rows')
     ap.add_argument('--strong', action='store_true', help='also run the 4320p strong-scaling case at N = 1 (always run for N > 1)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help="write the last timed picture's results (rank 0's band) as DIR/<name>.npy, to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the GPU path\'s results; --impl reference has none')
     rank = int(os.environ.get('RANK', '0')); world = int(os.environ.get('WORLD_SIZE', '1')); local = int(os.environ.get('LOCAL_RANK', '0'))
     PPS = max(1, args.pictures_per_step)
     u = units_per_picture()
@@ -746,6 +771,8 @@ def main():
         sampler.start()
     ms_total, launches = timed(step_resident, args.steps, max(3, args.warmup))
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(job, args.dump_outputs, V)
     ms_step = ms_total / args.steps
     ms_picture = ms_step / PPS
     value = units_picture_all * PPS / (ms_step * 1e-3)
@@ -1030,14 +1057,14 @@ def main():
                 par = eng.tu_par(n, n, 0, 0, BITDEPTH, QP, sign_hiding=True); rqp = VL.vvb_rdoq_par(57.3, 8, 0)
                 row = {'tus': int(cnt)}
                 for mult in (1, 16):
-                    d_c = torch.from_numpy(coef).cuda().repeat(mult, 1, 1); d_q = torch.zeros((cnt * mult, n, n), dtype=torch.int16, device='cuda')
+                    d_c = torch.from_numpy(coef).cuda().repeat(mult, 1, 1); d_rq = torch.zeros((cnt * mult, n, n), dtype=torch.int16, device='cuda')
                     d_s = torch.zeros(cnt * mult, dtype=torch.int32, device='cuda'); d_l = torch.zeros(cnt * mult, dtype=torch.int32, device='cuda')
                     t = time_launch(lambda: chk(lib.vvb_rdoq_dev(eng.h, ctypes.byref(par), ctypes.byref(rqp), ctypes.byref(rates), P_(d_c.data_ptr()), None, cnt * mult,
-                                                                 P_(d_q.data_ptr()), P_(d_s.data_ptr()), P_(d_l.data_ptr()))), reps=3)
+                                                                 P_(d_rq.data_ptr()), P_(d_s.data_ptr()), P_(d_l.data_ptr()))), reps=3)
                     row['ms_per_picture' if mult == 1 else 'ms_per_picture_at_16_pictures'] = t / mult
                     if mult == 1:
-                        q_dev = d_q.cpu().numpy(); l_dev = d_l.cpu().numpy()
-                    del d_c, d_q, d_s, d_l
+                        q_dev = d_rq.cpu().numpy(); l_dev = d_l.cpu().numpy()
+                    del d_c, d_rq, d_s, d_l
                 qq = np.zeros((cnt, n, n), dtype=np.int16); ss = np.zeros(cnt, dtype=np.int32); ll = np.zeros(cnt, dtype=np.int32)
                 t0 = time.perf_counter()
                 dq_oracle().orc_rdoq(n, n, BITDEPTH, QP, 0, 0, 0, 1, 57.3, 8, P_np(rates_flat), P_np(coef), cnt, P_np(qq), P_np(ss), P_np(ll))

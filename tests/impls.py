@@ -3,7 +3,7 @@ loops (tests/cases.py) drive: oracle-vs-golden, oracle-vs-reference and (tests/t
 import ctypes
 import numpy as np
 import cases as C
-from _libs import oracle, refshim, P, PO
+from _libs import answered, oracle, refshim, P, PO
 
 I32 = ctypes.c_int32
 
@@ -185,8 +185,9 @@ def run_rt(impl, rows, q, reco, meta):
     return bad
 
 
-def mctf_apply_expected(L, prefix, case, tap4, planar, opt=None):
-    """filtered picture [H][W] through the oracle (prefix 'orc') or the reference probe (prefix 'refshim', opt = 0/1), block by block"""
+def mctf_apply_expected(L, prefix, case, tap4, planar, opt=None, known=None):
+    """filtered picture [H][W] through the oracle (prefix 'orc') or the reference probe (prefix 'refshim', opt = 0/1), block by block;
+    `known` (bool [H][W]) is cleared over the blocks whose reference values a replayed probe could not give (see _libs.answered)"""
     S = case['stride']; m = case['margin']; W = case['W']; H = case['H']; bs = case['bs']; base = m * S + m
     out = np.zeros((H, W), dtype=np.int16)
     n = case['num_refs']
@@ -203,6 +204,8 @@ def mctf_apply_expected(L, prefix, case, tap4, planar, opt=None):
             else:
                 L.refshim_mctf_finalize_block(opt, PO(case['org'], base), S, ptrs, S, n, P(mv4), W, H, bx, by, w, h, case['bd'], tap4, planar, P(case['strengths']),
                                               ctypes.c_double(case['ws']), ctypes.c_double(case['sigma']), P(out), W)
+                if known is not None and not answered(out):
+                    known[by:by + h, bx:bx + w] = False
     return out
 
 

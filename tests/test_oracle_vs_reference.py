@@ -1,12 +1,17 @@
-"""CPU-only, build container only (skipped where oracle/_ref is absent): a wider random sweep of the oracle
-against the LIVE reference, scalar and AVX2, in the style of test/vvenc_unit_test (tolerance 0)."""
+"""CPU-only: a wider random sweep of the oracle against the reference, scalar and AVX2, in the style of test/vvenc_unit_test (tolerance 0).
+The reference answers through oracle/_ref where it is built, else from its recorded calls (tests/golden/refshim, see _libs.refshim)."""
 import numpy as np
 import pytest
 import cases as C
 import impls
-from _libs import have_ref
+from _libs import answered, have_ref, have_ref_results, refshim_reset
 
-pytestmark = pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not have_ref_results('test_oracle_vs_reference'), reason="neither oracle/_ref nor a recording of its calls")
+
+
+@pytest.fixture(autouse=True)
+def _fresh_refshim_replay():
+    refshim_reset()
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -40,7 +45,7 @@ def test_transform_quant_sweep(opt):
                 resi = rs.randint(-amp, amp + 1, size=(h, st)).astype(np.int16)
                 qp = int(rs.randint(0, 64)); irap = int(rs.randint(0, 2))
                 a = O.transform_quant(th, tv, resi, st, w, h, 10, qp, irap); b = R.transform_quant(th, tv, resi, st, w, h, 10, qp, irap)
-                assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and a[2:4] == b[2:4], (th, tv, w, h, qp, irap)
+                assert (not answered(b[0], b[1]) or np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])) and a[2:4] == b[2:4], (th, tv, w, h, qp, irap)
                 for dq in (0, 1):
                     assert O.need_rdoq(a[0], w, h, 10, qp, dq) == R.need_rdoq(a[0], w, h, 10, qp, dq)
 
@@ -59,8 +64,9 @@ def test_fwd_core_like_reference_unit_test():
             src = C.aligned((line, tr), np.int32); src[:] = rs.randint(-1024, 1024, size=(line, tr))
             d1 = C.aligned((tr, line), np.int32); d2 = C.aligned((tr, line), np.int32)
             R.refshim_fwd_core(tr, P(tc), P(src), P(d1), line, red, cut, shift); O.orc_fwd_core(tr, P(tc), P(src), P(d2), line, red, cut, shift)
+            known = answered(d1)
             d1 = d1[:, :red]; d2 = d2[:, :red]      # columns past reducedLine are unspecified (vvenc_unit_test.cpp:1117-1119)
-            assert np.array_equal(d1, d2), (tr, line, red, cut, shift)
+            assert not known or np.array_equal(d1, d2), (tr, line, red, cut, shift)
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -86,8 +92,10 @@ def test_affine(opt):
         w, h, ps, ds, six, seed = [int(v) for v in row]
         pred, resi, gx, gy = C.affine_inputs(row)
         for vert in (0, 1):
-            assert np.array_equal(O.sobel(vert, pred, ps, ds, w, h), R.sobel(vert, pred, ps, ds, w, h))
-        assert np.array_equal(O.equal_coeff(six, resi, ps, gx, gy, ds, w, h), R.equal_coeff(six, resi, ps, gx, gy, ds, w, h))
+            r = R.sobel(vert, pred, ps, ds, w, h)
+            assert not answered(r) or np.array_equal(O.sobel(vert, pred, ps, ds, w, h), r)
+        r = R.equal_coeff(six, resi, ps, gx, gy, ds, w, h)
+        assert not answered(r) or np.array_equal(O.equal_coeff(six, resi, ps, gx, gy, ds, w, h), r)
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -96,7 +104,7 @@ def test_full_search_with_tables(opt):
     sc = C.search_case(seed=991)
     for ss in (0, 1):
         a, ta = O.full_search(sc, ss, True); b, tb = R.full_search(sc, ss, True)
-        assert np.array_equal(a, b) and np.array_equal(ta, tb)
+        assert not answered(b, tb) or np.array_equal(a, b) and np.array_equal(ta, tb)
 
 
 def test_tables_match_reference():
@@ -108,12 +116,12 @@ def test_tables_match_reference():
     for (t, N), m in g.matrices().items():
         ref = np.zeros((N, N), dtype=np.int16)
         assert R.refshim_tr_matrix(t, N, P(ref)) == 0
-        assert np.array_equal(ref, m), (t, N)
+        assert not answered(ref) or np.array_equal(ref, m), (t, N)
     for w in (4, 8, 16, 32, 64):
         for h in (4, 8, 16, 32, 64):
             a = np.zeros(1024, dtype=np.int32); b = np.zeros(1024, dtype=np.int32)
             from _libs import oracle
-            assert R.refshim_scan_order(w, h, P(a)) == oracle().orc_scan_order(w, h, P(b)) and np.array_equal(a, b)
+            assert R.refshim_scan_order(w, h, P(a)) == oracle().orc_scan_order(w, h, P(b)) and (not answered(a) or np.array_equal(a, b))
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -130,7 +138,7 @@ def test_inverse_path_sweep(opt):
                     q = rs.randint(-amp - 1, amp + 1, size=(h, w)).astype(np.int16)
                     q[rs.rand(h, w) < 0.5] = 0
                     a = O.inv_transform_quant(th, tv, q, w, h, bd, qp, st); b = R.inv_transform_quant(th, tv, q, w, h, bd, qp, st)
-                    assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), (th, tv, w, h, bd, qp)
+                    assert not answered(b[0]) or np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), (th, tv, w, h, bd, qp)
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -147,7 +155,7 @@ def test_tu_roundtrip_sweep(opt):
                 pred = np.zeros((h, ps), dtype=np.int16)
                 pred[:, :w] = np.clip(org[:, :w] + rs.randint(-amp, amp + 1, size=(h, w)), 0, 1023)
                 a = O.tu_roundtrip(th, tv, org, so, pred, ps, w, h, 10, qp, irap); b = R.tu_roundtrip(th, tv, org, so, pred, ps, w, h, 10, qp, irap)
-                assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and a[2] == b[2], (th, tv, w, h, qp, irap, a[2], b[2])
+                assert not answered(b[0], b[1]) or np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]) and a[2] == b[2], (th, tv, w, h, qp, irap, a[2], b[2])
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -159,8 +167,9 @@ def test_mctf_apply_stage(opt):
     for (seed, W, H, refs, bs, bd, tap4, planar) in C.MCTF_APPLY_CASES:
         case = C.mctf_apply_case(seed, W, H, 24, refs, bs, bd)
         a = impls.mctf_apply_expected(O, 'orc', case, tap4, planar)
-        b = impls.mctf_apply_expected(R, 'refshim', case, tap4, planar, opt)
-        assert np.array_equal(a, b), (seed, np.abs(a.astype(int) - b).max())
+        known = np.ones(a.shape, dtype=bool)
+        b = impls.mctf_apply_expected(R, 'refshim', case, tap4, planar, opt, known)
+        assert np.array_equal(a[known], b[known]), (seed, np.abs(a.astype(int) - b)[known].max())
         assert np.any(a != case['org'][24:24 + H, 24:24 + W])           # the filter does something
 
 
@@ -199,7 +208,7 @@ def test_two_pass_interpolation(opt):
                         d1 = np.zeros((h, w), np.int16); d2 = np.zeros((h, w), np.int16)
                         O.orc_if_two_pass(PO(src, 8 * S + 12), S, w, h, fx, fy, bd, rt, alt, P(d1), w)
                         R.refshim_if_two_pass(opt, PO(src, 8 * S + 12), S, w, h, fx, fy, bd, rt, alt, P(d2), w)
-                        assert np.array_equal(d1, d2), (bd, w, h, rt, alt, fx, fy)
+                        assert not answered(d2) or np.array_equal(d1, d2), (bd, w, h, rt, alt, fx, fy)
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -249,6 +258,8 @@ def test_mctf_apply_against_the_reference_member_function(opt):
         R.refshim_mctf_bilateral_filter(opt, P(org), ptrs, nrefs, P(np.ascontiguousarray(mv)), P(idx), W, H, 10, unit, qp, ctypes.c_double(overall), reorder, tap4,
                                         P(got), P(strg), ctypes.byref(sig))
         assert sig.value == 9.0 * (128.0 + 3.0 / 256.0 * qp * qp * qp)                      # 10 bit: bitDepthDiffWeighting = 1
+        if not answered(got, strg):
+            continue
         pad = 128
         case = dict(org=np.ascontiguousarray(np.pad(org, pad, mode='edge')), refs=[np.ascontiguousarray(np.pad(r, pad, mode='edge')) for r in refs],
                     stride=W + 2 * pad, margin=pad, W=W, H=H, mvs=mv, strengths=strg, ws=overall * 0.4, sigma=sig.value, bs=unit, bd=10, num_refs=nrefs)
@@ -422,7 +433,7 @@ def test_sign_bit_hiding_against_the_reference(opt):
                 continue
             coefO = np.zeros((h, w), dtype=np.int32); qO = np.zeros((h, w), dtype=np.int16); sO = ctypes.c_int32(); lO = ctypes.c_int32()
             assert O.orc_transform_quant_ex(th, tv, P(resi), st, w, h, bd, qp, irap, sh, P(coefO), P(qO), ctypes.byref(sO), ctypes.byref(lO)) == 0
-            assert np.array_equal(qO, qR) and sO.value == sR.value and lO.value == lR.value, (row, int((qO != qR).sum()), sO.value, sR.value, lO.value, lR.value)
+            assert (not answered(qR) or np.array_equal(qO, qR)) and sO.value == sR.value and lO.value == lR.value, (row, int((qO != qR).sum()), sO.value, sR.value, lO.value, lR.value)
             q0 = np.zeros((h, w), dtype=np.int16); s0 = ctypes.c_int32(); l0 = ctypes.c_int32()
             O.orc_transform_quant_ex(th, tv, P(resi), st, w, h, bd, qp, irap, 0, P(coefO), P(q0), ctypes.byref(s0), ctypes.byref(l0))
             changed += int(not np.array_equal(q0, qO)); moved_last += int(l0.value != lO.value); n += 1
@@ -452,8 +463,8 @@ def test_lfnst_forward_against_the_reference(opt):
                 assert R.refshim_transform_quant_lfnst(P(resi), w, w, h, 10, qp, irap, sh, mode, idx, P(cR), P(qR), ctypes.byref(sR), ctypes.byref(lR), ctypes.byref(nR), P(st)) == 0
                 cO = np.zeros((h, w), dtype=np.int32); qO = np.zeros((h, w), dtype=np.int16); sO = ctypes.c_int32(); lO = ctypes.c_int32()
                 assert O.orc_transform_quant_lfnst(P(resi), w, w, h, 10, qp, irap, sh, int(st[0]), idx, int(st[1]), P(cO), P(qO), ctypes.byref(sO), ctypes.byref(lO)) == 0
-                assert np.array_equal(cO, cR), (w, h, mode, idx, st, np.argwhere(cO != cR)[:4])
-                assert np.array_equal(qO, qR) and sO.value == sR.value and lO.value == lR.value, (w, h, mode, idx, qp, sh)
+                assert not answered(cR) or np.array_equal(cO, cR), (w, h, mode, idx, st, np.argwhere(cO != cR)[:4])
+                assert (not answered(qR) or np.array_equal(qO, qR)) and sO.value == sR.value and lO.value == lR.value, (w, h, mode, idx, qp, sh)
                 assert O.orc_need_rdoq(P(cO), w, h, 10, qp, 0) == nR.value
                 sets.add((int(st[0]), int(st[1]))); n += 1
     assert n == 288 and len(sets) >= 6, (n, sets)
@@ -469,7 +480,7 @@ def test_dep_quant_scan_tables_equal_the_reference_rom():
             nc = min(w, 32) * min(h, 32)
             a = np.zeros(nc * 24, np.uint8); b = np.zeros(nc * 16, np.uint8); c = np.zeros(nc * 24, np.uint8); d = np.zeros(nc * 16, np.uint8)
             assert R.refshim_dep_quant_tables(w, h, P(a), P(b)) == nc and O.orc_dep_quant_tables(w, h, P(c), P(d)) == nc
-            assert np.array_equal(a, c) and np.array_equal(b, d), (w, h)
+            assert not answered(a, b) or np.array_equal(a, c) and np.array_equal(b, d), (w, h)
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -502,13 +513,15 @@ def test_dep_quant_against_the_reference_member(opt):
                     qR = np.zeros((h, w), np.int16); sR = ctypes.c_int32(); lR = ctypes.c_int32(); rates = np.zeros(266, np.int32); kR = np.zeros(9, np.int64)
                     assert R.refshim_dep_quant(P(coef), w, h, bd, qp, mts, intra, lf, sbt, lam, thr, opt, int(rs.randint(17, 52)), trial % 3, P(qR), ctypes.byref(sR), ctypes.byref(lR),
                                                P(rates), P(kR)) == 0
+                    n += 1; nonzero += int(lR.value >= 0); big += int(np.abs(qR).max() > 127)
+                    if not answered(qR, rates, kR):                           # replay: levels, rate tables and constants of the recorded sample
+                        continue
                     kO = np.zeros(9, np.int64)
                     assert O.orc_dep_quant_constants(w, h, bd, qp, lam, thr, P(kO)) == 0 and np.array_equal(kO, kR), (w, h, bd, qp, lam, kO, kR)
                     qO = np.zeros((h, w), np.int16); sO = ctypes.c_int32(); lO = ctypes.c_int32()
                     assert O.orc_dep_quant(w, h, bd, qp, lam, thr, zo, lf, 1 - opt, P(rates), P(coef), 1, P(qO), ctypes.byref(sO), ctypes.byref(lO)) == 0
                     assert np.array_equal(qO, qR) and sO.value == sR.value and lO.value == lR.value, (w, h, bd, qp, lam, scale, mts, lf, sbt, int((qO != qR).sum()))
-                    n += 1; nonzero += int(lR.value >= 0); big += int(np.abs(qR).max() > 127)
-    assert n == 1050 and nonzero > 500 and big > 10, (n, nonzero, big)
+    assert n == 1050 and nonzero > 500 and (big > 10 or not have_ref()), (n, nonzero, big)      # big reads every level array: the live probe only
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -543,6 +556,9 @@ def test_rdoq_against_the_reference_member(opt):
                     qR = np.zeros((h, w), np.int16); sR = ctypes.c_int32(); lR = ctypes.c_int32(); rates = np.zeros(190, np.int32); kR = np.zeros(7, np.int32)
                     assert R.refshim_rdoq(comp, P(coef), w, h, bd, qp, intra, lf, sbt, sh, cb, lam, thr, int(rs.randint(17, 52)), trial % 3, P(qR), ctypes.byref(sR), ctypes.byref(lR),
                                           P(rates), P(kR)) == 0
+                    n += 1; nonzero += int(lR.value >= 0); hidden += int(sh and lR.value >= 0)
+                    if not answered(qR, rates, kR):
+                        continue
                     kO = np.zeros(7, np.int32)
                     assert O.orc_rdoq_constants(w, h, bd, qp, int(comp > 0), lf, sbt, thr, P(kO)) == 0 and np.array_equal(kO, kR), (w, h, bd, qp, comp, lf, sbt, kO, kR)
                     qO = np.zeros((h, w), np.int16); sO = ctypes.c_int32(); lO = ctypes.c_int32()
@@ -551,7 +567,6 @@ def test_rdoq_against_the_reference_member(opt):
                     q2 = np.zeros((h, w), np.int16); s2 = ctypes.c_int32(); l2 = ctypes.c_int32()        # the second engine (accumulated templates, cost tables)
                     assert O.orc_rdoq_v2(w, h, bd, qp, int(comp > 0), lf, sbt, sh, lam, thr, P(rates), P(coef), 1, P(q2), ctypes.byref(s2), ctypes.byref(l2)) == 0
                     assert np.array_equal(q2, qR) and s2.value == sR.value and l2.value == lR.value, ('engine 2', w, h, bd, qp, comp, lf, sbt, intra, sh, cb, lam, scale, int((q2 != qR).sum()))
-                    n += 1; nonzero += int(lR.value >= 0); hidden += int(sh and lR.value >= 0)
     R.refshim_set_simd(b'AVX2')
     assert n == 1050 and nonzero > 450 and hidden > 150, (n, nonzero, hidden)
 
@@ -583,14 +598,16 @@ def test_rdoq_ts_against_the_reference_member(opt):
                     comp = int(rs.randint(2)); intra = int(rs.randint(2)); delta = int(rs.choice([0, 0, 2])) if bd == 10 else 0
                     qR = np.zeros((h, w), np.int16); sR = ctypes.c_int32(); rates = np.zeros(44, np.int32); kR = np.zeros(3, np.int32); eR = ctypes.c_double()
                     assert R.refshim_rdoq_ts(comp, P(coef), w, h, bd, qp, delta, intra, lam, int(rs.randint(17, 52)), trial % 3, P(qR), ctypes.byref(sR), P(rates), P(kR), ctypes.byref(eR)) == 0
+                    n += 1; nonzero += int(sR.value > 0); big += int(np.abs(qR).max() > 9)
+                    if not answered(qR, rates):
+                        continue
                     kO = np.zeros(3, np.int32); eO = ctypes.c_double()
                     assert O.orc_rdoq_ts_constants(w, h, bd, qp, delta, P(kO), ctypes.byref(eO)) == 0 and np.array_equal(kO, kR) and eO.value == eR.value, (w, h, bd, qp, delta, kO, kR)
                     qO = np.zeros((h, w), np.int16); sO = ctypes.c_int32()
                     assert O.orc_rdoq_ts(w, h, bd, qp, delta, lam, P(rates), P(coef), 1, P(qO), ctypes.byref(sO)) == 0
                     assert np.array_equal(qO, qR) and sO.value == sR.value, (w, h, bd, qp, comp, intra, delta, lam, amp, kind, int((qO != qR).sum()))
-                    n += 1; nonzero += int(sR.value > 0); big += int(np.abs(qR).max() > 9)
     R.refshim_set_simd(b'AVX2')
-    assert n == 1152 and nonzero > 600 and big > 150, (n, nonzero, big)
+    assert n == 1152 and nonzero > 600 and (big > 150 or not have_ref()), (n, nonzero, big)      # big reads every level array: the live probe only
 
 
 @pytest.mark.parametrize("opt", [0, 1])
@@ -618,10 +635,12 @@ def test_rdoq_bdpcm_against_the_reference_member(opt):
                     comp = int(rs.randint(2)); delta = int(rs.choice([0, 0, 2])) if bd == 10 else 0; dm = 1 + int(rs.randint(2))
                     qR = np.zeros((h, w), np.int16); sR = ctypes.c_int32(); rates = np.zeros(44, np.int32)
                     assert R.refshim_rdoq_bdpcm(comp, P(coef), w, h, bd, qp, delta, 1, dm, lam, int(rs.randint(17, 52)), trial % 3, P(qR), ctypes.byref(sR), P(rates)) == 0
+                    n += 1; nonzero += int(sR.value > 0)
+                    if not answered(qR, rates):
+                        continue
                     qO = np.zeros((h, w), np.int16); sO = ctypes.c_int32()
                     assert O.orc_rdoq_bdpcm(w, h, bd, qp, delta, dm, lam, P(rates), P(coef), 1, P(qO), ctypes.byref(sO)) == 0
                     assert np.array_equal(qO, qR) and sO.value == sR.value, (w, h, bd, qp, comp, delta, dm, lam, amp, kind, int((qO != qR).sum()))
-                    n += 1; nonzero += int(sR.value > 0)
     R.refshim_set_simd(b'AVX2')
     assert n == 1152 and nonzero > 700, (n, nonzero)
 
@@ -648,14 +667,14 @@ def test_transform_skip_and_chroma_against_the_reference(opt):
             assert O.orc_transform_quant_ts(P(resi), st, w, h, bd, qp, irap, sh, delta, P(cO), P(qO), ctypes.byref(sO), ctypes.byref(lO)) == 0
         else:
             assert O.orc_transform_quant_ex(0, 0, P(resi), st, w, h, bd, qp, irap, sh, P(cO), P(qO), ctypes.byref(sO), ctypes.byref(lO)) == 0
-        assert np.array_equal(cO, cR) and np.array_equal(qO, qR) and sO.value == sR.value and lO.value == lR.value, [int(v) for v in row]
+        assert (not answered(cR, qR) or np.array_equal(cO, cR) and np.array_equal(qO, qR)) and sO.value == sR.value and lO.value == lR.value, [int(v) for v in row]
         assert O.orc_need_rdoq_ex(P(cO), w, h, bd, qp, dq, ts, delta, comp) == nR.value, [int(v) for v in row]
         n += 1; nts += ts
         if ts and sR.value > 0:
             rR = np.zeros((h, st), np.int16); rO = np.zeros((h, st), np.int16); dR = np.zeros((h, w), np.int32); dO = np.zeros((h, w), np.int32)
             assert R.refshim_inv_transform_quant_ts(P(qR), w, h, bd, qp, delta, P(dR), P(rR), st) == 0
             assert O.orc_inv_transform_quant_ts(P(qR), w, h, bd, qp, delta, P(dO), P(rO), st) == 0
-            assert np.array_equal(dR, dO) and np.array_equal(rR[:, :w], rO[:, :w]), [int(v) for v in row]
+            assert not answered(dR, rR) or np.array_equal(dR, dO) and np.array_equal(rR[:, :w], rO[:, :w]), [int(v) for v in row]
             ninv += 1
     assert n == 220 and nts >= 80 and ninv > 40, (n, nts, ninv)
 
@@ -671,7 +690,7 @@ def test_dep_quant_chroma_against_the_reference_member(opt):
             nc = min(w, 32) * min(h, 32)
             a = np.zeros(nc * 24, np.uint8); b = np.zeros(nc * 16, np.uint8); c = np.zeros(nc * 24, np.uint8); d = np.zeros(nc * 16, np.uint8)
             assert R.refshim_dep_quant_tables_ex(1, w, h, P(a), P(b)) == nc and O.orc_dep_quant_tables_ex(1, w, h, P(c), P(d)) == nc
-            assert np.array_equal(a, c) and np.array_equal(b, d), (w, h)
+            assert not answered(a, b) or np.array_equal(a, c) and np.array_equal(b, d), (w, h)
     rs = np.random.RandomState(700 + opt); n = 0; nz = 0
     for (w, h) in [(4, 4), (8, 8), (16, 16), (32, 32), (8, 4), (4, 16), (32, 8), (16, 32), (64, 64), (16, 4)]:
         for bd in (10, 8):
@@ -684,10 +703,12 @@ def test_dep_quant_chroma_against_the_reference_member(opt):
                     if h > 32: coef[32:, :] = 0
                     q = np.zeros((h, w), np.int16); s = ctypes.c_int32(); l = ctypes.c_int32(); rates = np.zeros(266, np.int32)
                     assert R.refshim_dep_quant_comp(1, P(coef), w, h, bd, qp, 0, int(rs.randint(2)), 0, 0, lam, 8, opt, int(rs.randint(17, 52)), trial % 3, P(q), ctypes.byref(s), ctypes.byref(l), P(rates), None) == 0
+                    n += 1; nz += int(l.value >= 0)
+                    if not answered(q, rates):
+                        continue
                     q2 = np.zeros((h, w), np.int16); s2 = ctypes.c_int32(); l2 = ctypes.c_int32()
                     assert O.orc_dep_quant_chroma(w, h, bd, qp, lam, 8, 0, 1 - opt, P(rates), P(coef), 1, P(q2), ctypes.byref(s2), ctypes.byref(l2)) == 0
                     assert np.array_equal(q, q2) and s.value == s2.value and l.value == l2.value, (w, h, bd, qp, lam, scale)
-                    n += 1; nz += int(l.value >= 0)
     assert n == 400 and nz > 150, (n, nz)
 
 
@@ -706,7 +727,7 @@ def test_dep_quant_dequantiser_against_the_reference(opt):
         cR = np.zeros((h, w), np.int32); rR = np.zeros((h, w), np.int16); cO = np.zeros((h, w), np.int32); rO = np.zeros((h, w), np.int16)
         assert R.refshim_inv_transform_quant_dq(th, tv, P(q), last, w, h, bd, qp, P(cR), P(rR), w) == 0
         assert O.orc_inv_transform_quant_dq(th, tv, P(q), w, h, bd, qp, P(cO), P(rO), w) == 0
-        assert np.array_equal(cR, cO) and np.array_equal(rR, rO), [int(v) for v in row]
+        assert not answered(cR, rR) or np.array_equal(cR, cO) and np.array_equal(rR, rO), [int(v) for v in row]
         n += 1
     assert n == 168
 
@@ -729,8 +750,8 @@ def test_lfnst_inverse_against_the_reference(opt):
         assert R.refshim_inv_transform_quant_lfnst(P(q), w, h, bd, qp, dq, last, mode, idx, P(cR), P(rR), w, P(st)) == 0
         cO = np.zeros((h, w), np.int32); rO = np.zeros((h, w), np.int16)
         assert O.orc_inv_transform_quant_lfnst(P(q), w, h, bd, qp, dq, int(st[0]), idx, int(st[1]), P(cO), P(rO), w) == 0
-        assert np.array_equal(rR, rO), [int(v) for v in row]
+        assert not answered(rR) or np.array_equal(rR, rO), [int(v) for v in row]
         k = 8 if (w >= 8 and h >= 8) else 4
-        assert np.array_equal(cR[:k, :k], cO[:k, :k]), [int(v) for v in row]       # what xIT reads
+        assert not answered(cR) or np.array_equal(cR[:k, :k], cO[:k, :k]), [int(v) for v in row]       # what xIT reads
         sets.add((int(st[0]), int(st[1]))); n += 1; nz += int(rR.any())
-    assert n == 288 and len(sets) >= 6 and nz > 200, (n, sets, nz)
+    assert n == 288 and len(sets) >= 6 and (nz > 200 or not have_ref()), (n, sets, nz)      # nz reads every residual: the live probe only

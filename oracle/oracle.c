@@ -617,6 +617,28 @@ int orc_transform_quant( int trHor, int trVer, const Pel* resi, int stride, int 
   if( orc_fwd_transform( trHor, trVer, resi, stride, w, h, bitDepth, coef ) ) return -1;
   return orc_quant( coef, w, h, bitDepth, qp, isIRAP, q, absSum, lastPos );
 }
+/* list form over the blocks of two planes: TU i takes the residual org(x, y) - ref(x + dx, y + dy) of pos[i] = { x, y, dx, dy }, then
+ * orc_transform_quant and orc_need_rdoq on its coefficients; q holds n compact w x h level blocks */
+int orc_transform_quant_blocks( int trHor, int trVer, const Pel* orgPlane, int so, const Pel* refPlane, int sr, const int32_t* pos, int n, int w, int h,
+                                int bitDepth, int qp, int isIRAP, int depQuant, int16_t* q, int32_t* absSum, int32_t* lastPos, uint8_t* needRdoq )
+{
+  Pel* resi = (Pel*) malloc( sizeof( Pel ) * w * h );
+  int32_t* coef = (int32_t*) malloc( sizeof( int32_t ) * w * h );
+  int rc = 0;
+  for( int i = 0; i < n && !rc; i++ )
+  {
+    const int32_t* d = pos + 4 * (size_t) i;
+    const Pel* o = orgPlane + (ptrdiff_t) d[1] * so + d[0];
+    const Pel* r = refPlane + (ptrdiff_t)( d[1] + d[3] ) * sr + d[0] + d[2];
+    for( int y = 0; y < h; y++ )
+      for( int x = 0; x < w; x++ ) resi[y * w + x] = (Pel)( o[y * so + x] - r[y * sr + x] );
+    rc = orc_transform_quant( trHor, trVer, resi, w, w, h, bitDepth, qp, isIRAP, coef, q + (size_t) i * w * h, absSum + i, lastPos + i );
+    needRdoq[i] = (uint8_t) orc_need_rdoq( coef, w, h, bitDepth, qp, depQuant );
+  }
+  free( resi ); free( coef );
+  return rc;
+}
+
 /* same with slice->signDataHidingEnabled (Quant.cpp:748) */
 int orc_transform_quant_ex( int trHor, int trVer, const Pel* resi, int stride, int w, int h, int bitDepth, int qp, int isIRAP, int signHiding,
                             int32_t* coef, int16_t* q, int32_t* absSum, int32_t* lastPos )
